@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- JPEG encode throughput of the B200 path (and of the CPU reference arm).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--config 1..5]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--config 1..5] [--dump-outputs DIR]
 
 Headline workload (BASELINE.json configs[1] = SURVEY 8d config 2, the one the metric is quoted on; --config picks another):
     synthetic 1920x1080 RGB, batch of 256 per GPU, IJG quality 75, 4:2:0.
@@ -92,6 +92,26 @@ def cpu_encode_rate(images, qmode, quality, sub, threads, min_seconds=2.0, max_s
     for t in ths: t.start()
     for t in ths: t.join()
     return done[0] * mp / t_end[0], kind, done[0], t_end[0]
+
+
+def dump_outputs(out_dir, files, budget=64_000_000):
+    """--dump-outputs: what a caller of the timed path receives, the JPEG files of its last step, for comparing two builds.
+    encoded_sizes.npy holds every file's length (-1: not encoded); encoded_files.npy the byte values (float32) of whole files,
+    taken in a fixed seeded order while everything fits `budget` bytes; encoded_files_index.npy which files those are."""
+    os.makedirs(out_dir, exist_ok=True)
+    sizes = np.array([len(f) if f is not None else -1 for f in files], np.float64)
+    room = budget - sizes.nbytes
+    pick = []
+    for i in np.random.default_rng(0).permutation(len(files)):
+        need = 4 * sizes[i] + 8
+        if sizes[i] > 0 and need <= room:
+            pick.append(int(i))
+            room -= need
+    pick.sort()
+    data = np.frombuffer(b"".join(files[i] for i in pick), np.uint8).astype(np.float32)
+    np.save(os.path.join(out_dir, "encoded_sizes.npy"), sizes)
+    np.save(os.path.join(out_dir, "encoded_files_index.npy"), np.array(pick, np.float64))
+    np.save(os.path.join(out_dir, "encoded_files.npy"), data)
 
 
 def run_reference(args):
@@ -358,6 +378,8 @@ def run_ours(args):
     cfg = CONFIGS[K]
     with ClockSampler(local) as clk:
         head, plan, pixels = measure_config(K, args.steps, args.warmup, check=2, keep=True)
+    if args.dump_outputs and plan is not None and rank == 0:
+        dump_outputs(args.dump_outputs, plan.fetch(sptr))
     launches = plan.launches if plan is not None else 0     # per quantiser group: transform + entropy + plan_chunks + count_ff + scan_groups + stuff
     clocks = clk.summary()
     ms_step = head["ms_per_step"]
@@ -517,11 +539,11 @@ def run_ours(args):
                 t0 = time.perf_counter()
                 dec_px = jg.decode_batch(rfiles, alloc=alloc)                            # untimed: chunks pipelined over three host threads
                 dec_call = (time.perf_counter() - t0) * 1e3
-                ok = all(np.array_equal(dec_px[i], oracle.ref_decode(rfiles[i])) for i in (0, n_img - 1))
+                ok = all(np.array_equal(dec_px[i], oracle.ref_decode(rfiles[i])) for i in (0, n_img - 1)) if oracle.have_ref() else None
                 decode[key] = {"workload": "the same %d images, IJG q75 4:2:0, %s" % (n_img, "one restart interval per 24 blocks" if flags else
                                                                                      "ordinary files (no restart markers): self-synchronising subsequences"),
                                "value": round(n_img * W * H / 1e6 / (dec_ms * 1e-3), 1), "unit": UNIT, "kernels_ms": round(dec_ms, 3),
-                               "call_ms_host_files_to_host_pixels": round(dec_call, 1), "first_call_ms": round(dec_first, 1), "host_buffers": "files pageable, pixels pinned", "pixels_identical_to_reference_decoder": bool(ok)}
+                               "call_ms_host_files_to_host_pixels": round(dec_call, 1), "first_call_ms": round(dec_first, 1), "host_buffers": "files pageable, pixels pinned", "pixels_identical_to_reference_decoder": ok}
                 del dec_px, pinned
             except Exception as e:
                 decode[key] = {"error": repr(e)}
@@ -588,7 +610,12 @@ def main():
     ap.add_argument("--no-cpu", action="store_true", help="skip the cpu_baseline leg")
     ap.add_argument("--no-twin", action="store_true", help="skip the decode legs")
     ap.add_argument("--no-configs", action="store_true", help="skip the per-configuration table")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the JPEG files of the last timed step to DIR as .npy (see dump_outputs)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs needs --impl ours")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
     if args.impl == "reference":
         return run_reference(args)

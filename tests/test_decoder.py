@@ -1,6 +1,6 @@
 """The decoder (SURVEY 8f rank 1): the product's decoder SOURCE (jpeg_decode.cuh / jpeg_decode_host.cpp) run on the
-CPU, where one loop iteration is what one GPU thread executes, against the reference's NanoJPEG (oracle/_ref)
-and the committed fixture.  Bit-exact pixels are the bar.  The GPU run of the same code is in test_gpu_parity.py."""
+CPU, where one loop iteration is what one GPU thread executes, against the reference's NanoJPEG (its recorded answers,
+tests/golden/ref_digests.json) and the committed fixture.  Bit-exact pixels are the bar.  The GPU run of the same code is in test_gpu_parity.py."""
 import io
 import os
 
@@ -9,6 +9,7 @@ import pytest
 
 import oracle
 from tests.emu.emu import emu_decode, emu_set_round_order
+from tests.helpers import pixel_digest, ref_decoded
 
 GOLDEN = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden")
 
@@ -27,9 +28,9 @@ def test_reference_fixture_decodes_to_the_committed_pixels():
 def test_decodes_our_own_streams_like_the_reference_decoder(w, h, nc, qm, q, sub, rst):
     img = oracle.synth_image(w, h, nc, kind="noise" if (w, h) == (64, 64) else "photo")
     jpeg = oracle.oracle_encode(img, qm, q, sub, restart=rst)
-    want = oracle.ref_decode(jpeg)
+    want = ref_decoded(jpeg)
     got = emu_decode(jpeg)
-    assert want is not None and isinstance(got, np.ndarray) and np.array_equal(got, want)
+    assert want is not None and pixel_digest(got) == want
 
 
 def test_decodes_other_encoders_files():
@@ -40,16 +41,16 @@ def test_decodes_other_encoders_files():
     for im, kw in [(rgb, dict(subsampling=0)), (rgb, dict(subsampling=1)), (rgb, dict(subsampling=2)), (rgb, dict(subsampling=2, quality=30, optimize=True)),
                    (gray, dict(quality=85)), (gray, dict(quality=95, optimize=True))]:
         b = io.BytesIO(); im.save(b, "JPEG", **kw)
-        want = oracle.ref_decode(b.getvalue())
+        want = ref_decoded(b.getvalue())
         got = emu_decode(b.getvalue())
-        assert want is not None and isinstance(got, np.ndarray) and np.array_equal(got, want), kw
+        assert want is not None and pixel_digest(got) == want, kw
 
 
 def test_rejects_what_the_reference_rejects():
     from PIL import Image
     assert emu_decode(b"\x00\x01\x02\x03") == 1                                    # NJ_NO_JPEG
     b = io.BytesIO(); Image.fromarray(oracle.synth_image(64, 48, 3)).save(b, "JPEG", progressive=True)
-    assert oracle.ref_decode(b.getvalue()) is None and emu_decode(b.getvalue()) == 2    # progressive: NJ_UNSUPPORTED
+    assert ref_decoded(b.getvalue()) is None and emu_decode(b.getvalue()) == 2    # progressive: NJ_UNSUPPORTED
     good = oracle.oracle_encode(oracle.synth_image(40, 40, 3), 0, 3, 0)
     assert emu_decode(good[:300]) == 5                                             # truncated in the tables: NJ_SYNTAX_ERROR
 
@@ -72,9 +73,9 @@ def test_decodes_foreign_restart_streams_and_411():
     b = io.BytesIO(); Image.fromarray(img).save(b, "JPEG", subsampling="4:1:1", quality=80)
     files.append(b.getvalue())
     for i, f in enumerate(files):
-        want = oracle.ref_decode(f)
+        want = ref_decoded(f)
         got = emu_decode(f)
-        assert want is not None and isinstance(got, np.ndarray) and np.array_equal(got, want), i
+        assert want is not None and pixel_digest(got) == want, i
 
 
 # ---- restart-free scans: the subsequence (self-synchronising) decode --------------------------------------------
@@ -86,18 +87,18 @@ def test_subsequence_decode_equals_the_reference_decoder(w, h, nc, qm, q, sub):
     threads that have nothing to decode, stuffed bytes on the cuts): same pixels as njDecode, whatever the size."""
     img = oracle.synth_image(w, h, nc, kind="noise" if (w, h) == (64, 64) else "photo")
     jpeg = oracle.oracle_encode(img, qm, q, sub)
-    want = oracle.ref_decode(jpeg)
+    want = ref_decoded(jpeg)
     assert want is not None
     try:
         for order in (0, 1, 2, 3):               # the threads of a round in different orders / racing host threads (records are updated in place)
             emu_set_round_order(order)
             for sub_log2 in (2, 3, 5, 7):
                 got, rounds = emu_decode(jpeg, sub_log2, want_rounds=True)
-                assert isinstance(got, np.ndarray) and np.array_equal(got, want), (order, sub_log2)
+                assert pixel_digest(got) == want, (order, sub_log2)
                 assert rounds >= 2
     finally:
         emu_set_round_order(0)
-    assert np.array_equal(emu_decode(jpeg, 0), want)              # and the one-thread path still agrees
+    assert pixel_digest(emu_decode(jpeg, 0)) == want              # and the one-thread path still agrees
 
 
 def test_subsequence_decode_is_the_default_for_restart_free_files():
@@ -119,10 +120,10 @@ def test_subsequence_decode_of_other_encoders_files():
     for im, kw in [(rgb, dict(subsampling=0, quality=95)), (rgb, dict(subsampling=1)), (rgb, dict(subsampling=2, quality=30, optimize=True)),
                    (rgb, dict(subsampling="4:1:1", quality=80)), (gray, dict(quality=95, optimize=True))]:
         b = io.BytesIO(); im.save(b, "JPEG", **kw)
-        want = oracle.ref_decode(b.getvalue())
+        want = ref_decoded(b.getvalue())
         for sub_log2 in (3, 5, -1):
             got = emu_decode(b.getvalue(), sub_log2)
-            assert want is not None and isinstance(got, np.ndarray) and np.array_equal(got, want), (kw, sub_log2)
+            assert want is not None and pixel_digest(got) == want, (kw, sub_log2)
 
 
 def test_subsequence_decode_of_damaged_scans_agrees_with_the_one_thread_path():
@@ -190,13 +191,13 @@ def test_subsequence_decode_random_differential():
                 else:
                     Image.fromarray(img).save(b, "JPEG", subsampling=[0, 1, 2, "4:1:1"][int(rng.integers(0, 4))], **kw)
                 f = b.getvalue()
-            want = oracle.ref_decode(f)
+            want = ref_decoded(f)
             if want is None:
                 continue
             emu_set_round_order(int(rng.integers(0, 4)))
             sub_log2 = int(rng.integers(2, 8))
             got = emu_decode(f, sub_log2)
-            assert isinstance(got, np.ndarray) and np.array_equal(got, want), (it, w, h, sub_log2)
+            assert pixel_digest(got) == want, (it, w, h, sub_log2)
             checked += 1
     finally:
         emu_set_round_order(0)
